@@ -2,7 +2,7 @@
 """bench.py — decode tokens/s of the sync speculative-decoding hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu]
-                    [--workload 70b|8b|qwen32b|tiny] [--temp T] [--lm-scale S]
+                    [--workload 70b|8b|qwen32b|tiny] [--temp T] [--lm-scale S] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: K_spec+1 draft forwards -> one (K_spec+1)-token target
 forward -> accept/reject+resample.  Workload (N=1 default): Llama-3.1-70B target + Llama-3.2-1B draft, k=6, b=1,
@@ -210,8 +210,10 @@ def run_ours(args):
         e1.record()
         sync_all()
     ms_dev = e0.elapsed_time(e1)
-    _, tot1, _ = runner.fetch(1)
+    last_spec, tot1, last_rec = runner.fetch(1)
     dev_log = runner.resident_log(0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, runner, last_spec, tot1, last_rec, dev_log)
     launches = runner.launch_count - l0
     toks_dev = int(tot1[0] - tot0[0])
     if world > 1:
@@ -320,6 +322,21 @@ def run_ours(args):
             dist.destroy_process_group()
         except Exception:
             pass
+
+
+def dump_outputs(out_dir, runner, spec, total, rec, log):
+    """What the timed device-resident loop handed back after its last step, as .npy files (float64 for token ids and
+    counts, float32 for logits) so that two builds can be compared output for output on the same seeded inputs:
+    that step's speculations [1, K+1], the running count of emitted tokens, the recovery token, every token emitted
+    since the prefill, and the target [1, K+1, V] and draft [1, K, V] logits of that step (about 7 MB at V = 128256)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"speculations": spec.astype(np.float64), "tokens_total": total.astype(np.float64),
+              "recovery": rec.astype(np.float64), "emitted_tokens": np.asarray(log, dtype=np.float64),
+              "logits_target": runner.logits_p(1).float().cpu().numpy(),
+              "logits_draft": runner.logits_q(1).float().cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def gemm_roofline(runner, peak):
@@ -463,6 +480,8 @@ def main():
     ap.add_argument("--prompt-len", type=int, default=128)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-pdl", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":

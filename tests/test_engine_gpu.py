@@ -386,9 +386,9 @@ def test_spec_steps_across_the_draft_path_switch_match_oracle():
     ctx, rec = len(prompt), rec_o[0]
     launches = []
     for step in range(10):
-        n0 = r.launch_count()
+        n0 = r.launch_count
         toks, nacc, nrec = r.spec_step([ctx], [rec], [bt[0].tolist()], [bt[0].tolist()], [0.0], [0.0])
-        launches.append(r.launch_count() - n0)
+        launches.append(r.launch_count - n0)
         spec = torch.from_numpy(toks)
         lp_o, lq_o = s.spec_step_forced(spec)
         torch.testing.assert_close(r.logits_p(1).cpu().float(), lp_o.float(), atol=0.08, rtol=0.03)

@@ -1,21 +1,20 @@
 """The reference's OWN acceptance harness (bench/bench.py, unmodified, SURVEY §2 item 19) driven on top of the
 ssd_b200 host engine through the `ssd` compat shim — on CPU, with the device runner replaced by a deterministic test
-double.  Checks the drop-in boundary end to end: `import ssd.paths`, `from ssd import LLM, SamplingParams`,
-`from ssd.engine.llm_engine import METRICS`, the kwargs of `create_llm_kwargs`, `generate()`'s return value, the sweep
-path that pokes `llm.config.max_num_seqs` / `llm.scheduler.max_num_seqs`, and the scheduler / block-manager bookkeeping
-under random accept lengths.  Skipped where the reference checkout is absent (the GPU box)."""
+double.  The calls that harness makes into the engine (the model and the kwargs of `create_llm_kwargs`, the
+`llm.config.max_num_seqs` / `llm.scheduler.max_num_seqs` pokes of its sweep path, the METRICS reset, the prompts and
+SamplingParams handed to `generate()`) were recorded from a run of the unmodified harness into
+tests/golden/reference_bench_calls.json (oracle/gen_harness_golden.py); the tests replay them through `import ssd.paths`,
+`from ssd import LLM, SamplingParams`, `from ssd.engine.llm_engine import METRICS`, and check `generate()`'s return
+value and the scheduler / block-manager bookkeeping under random accept lengths."""
 import importlib
 import json
 import os
-import runpy
 import sys
 import types
 
 import numpy as np
-import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "bench")), reason="reference checkout not present")
+CALLS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_bench_calls.json")
 
 V = 128256
 
@@ -82,7 +81,9 @@ def _make_hf_cache(root):
         os.rename(made, os.path.join(snap, "synthetic"))
 
 
-def _run_bench(tmp_path, monkeypatch, argv):
+def engine_env(tmp_path, monkeypatch):
+    """SSD_HF_CACHE with the synthetic Llama 8B / 1B pair, the `ssd` compat shim, a wandb stub and FakeRunner in place
+    of the device runner.  Returns {"runner", "config"}, filled when the engine is built."""
     monkeypatch.setenv("SSD_HF_CACHE", str(tmp_path))
     monkeypatch.setenv("SSD_DATASET_DIR", str(tmp_path / "datasets"))
     _make_hf_cache(str(tmp_path))
@@ -103,27 +104,61 @@ def _run_bench(tmp_path, monkeypatch, argv):
 
     import ssd_b200.loader as loader
     monkeypatch.setattr(loader, "build_runner", fake_build_runner)
-    captured = {}
+    return fake
+
+
+def spy_engine(monkeypatch, cache_dir):
+    """Records every LLMEngine construction and generate() call: the calls as made (paths relative to `cache_dir`), and
+    what generate() returned."""
+    import dataclasses
+
     import ssd_b200.engine.llm_engine as eng
-    orig_generate = eng.LLMEngine.generate
+    calls, captured = {"runs": []}, {"runs": []}
+    orig_init, orig_generate = eng.LLMEngine.__init__, eng.LLMEngine.generate
+    rel = lambda p: os.path.relpath(p, cache_dir) if isinstance(p, str) and p.startswith(str(cache_dir)) else p
+
+    def spy_init(self, model, **kwargs):
+        calls["model"], calls["llm_kwargs"] = rel(model), {k: rel(v) for k, v in kwargs.items()}
+        orig_init(self, model, **kwargs)
 
     def spy_generate(self, prompts, sampling_params, use_tqdm=True, stream_callback=None):
+        calls["runs"].append({"config_max_num_seqs": self.config.max_num_seqs,
+                              "scheduler_max_num_seqs": self.scheduler.max_num_seqs, "prompts": [list(p) for p in prompts],
+                              "sampling_params": [dataclasses.asdict(sp) for sp in sampling_params]})
         outs, metrics = orig_generate(self, prompts, sampling_params, use_tqdm=False, stream_callback=stream_callback)
-        captured.setdefault("runs", []).append((prompts, outs, {k: (list(v) if isinstance(v, list) else v) for k, v in metrics.items()}))
+        captured["runs"].append((prompts, outs, {k: (list(v) if isinstance(v, list) else v) for k, v in metrics.items()}))
         return outs, metrics
 
+    monkeypatch.setattr(eng.LLMEngine, "__init__", spy_init)
     monkeypatch.setattr(eng.LLMEngine, "generate", spy_generate)
-    monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
-    monkeypatch.syspath_prepend(os.path.join(REF, "bench"))
-    with pytest.raises(SystemExit) as ex:
-        runpy.run_path(os.path.join(REF, "bench", "bench.py"), run_name="__main__")
-    assert ex.value.code == 0
+    return calls, captured
+
+
+def _run_bench(tmp_path, monkeypatch, name):
+    """Replay the recorded calls of the reference harness run `name` in the order it made them."""
+    with open(CALLS) as f:
+        rec = json.load(f)[name]
+    fake = engine_env(tmp_path, monkeypatch)
+    _, captured = spy_engine(monkeypatch, tmp_path)
+    import ssd.paths  # noqa: F401
+    from ssd import LLM, SamplingParams
+    from ssd.engine.llm_engine import METRICS
+    path = lambda p: os.path.join(ssd.paths.HF_CACHE_DIR, p) if p else p
+    llm = LLM(path(rec["model"]), **{**rec["llm_kwargs"], "draft": path(rec["llm_kwargs"]["draft"])})
+    for run in rec["runs"]:
+        llm.config.max_num_seqs = run["config_max_num_seqs"]
+        llm.scheduler.max_num_seqs = run["scheduler_max_num_seqs"]
+        for k, v in METRICS.items():
+            if isinstance(v, list):
+                v.clear()
+            else:
+                METRICS[k] = 0
+        llm.generate(run["prompts"], [SamplingParams(**sp) for sp in run["sampling_params"]])
     return captured, fake
 
 
 def test_reference_bench_py_runs_unmodified_on_the_engine(tmp_path, monkeypatch):
-    captured, fake = _run_bench(tmp_path, monkeypatch, ["--size", "8", "--spec", "--k", "6", "--random", "--numseqs", "5",
-                                                       "--input_len", "40", "--output_len", "60", "--b", "2"])
+    captured, fake = _run_bench(tmp_path, monkeypatch, "spec")
     cfg = fake["config"]
     assert cfg.speculate and cfg.speculate_k == 6 and cfg.jit_speculate and cfg.kvcache_block_size == 256
     assert cfg.max_num_seqs == 2 and cfg.max_model_len == 8192
@@ -144,9 +179,7 @@ def test_reference_bench_py_runs_unmodified_on_the_engine(tmp_path, monkeypatch)
 
 
 def test_reference_bench_py_sweep_and_autoregressive(tmp_path, monkeypatch):
-    captured, fake = _run_bench(tmp_path, monkeypatch, ["--size", "8", "--random", "--numseqs", "3", "--input_len", "16",
-                                                       "--output_len", "20", "--b", "2",
-                                                       "--sweep", json.dumps([{"b": 2, "temp": 0.5}, {"b": 1}])])
+    captured, fake = _run_bench(tmp_path, monkeypatch, "sweep")
     assert not fake["config"].speculate
     assert len(captured["runs"]) == 2
     for prompts, outs, metrics in captured["runs"]:
